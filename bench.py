@@ -20,6 +20,8 @@ Chains are independent trajectories (one b2s handle / CUDA stream each), the uni
   config3/4/5  : the other configurations of BASELINE.json, device-timed in the same run (open3d_slam_b200/benchmarks.py)
   cpu_baseline : the CPU oracle (oracle/, "port" of the reference's Open3D path) on a bounded sample, rank 0 only
   --impl reference : the same workload on the host cores through the oracle only (no GPU code on that path)
+  --dump-outputs DIR : after the timed steps, the last step's outputs as float64 DIR/<name>.npy (dump_last_step).  The inputs
+          are generated from fixed seeds, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -37,6 +39,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from (no __pycache__ either)
 
 from open3d_slam_b200 import synth  # noqa: E402
 from open3d_slam_b200 import workloads as W  # noqa: E402
@@ -46,6 +49,9 @@ UNIT = "registrations/s"
 WORKLOAD = "config2: scan-to-map odometry loop, synthetic 64x1024 LiDAR, voxel 0.1 m, Lua defaults, PointToPlaneIcp, steady-state map"
 SCAN_SETS = 8   # noise realisations of the lap; chain c replays set c % SCAN_SETS
 LAP = int(round(synth.loop_length() / 0.5))   # scans per lap of the closed loop (118)
+RESULT_SLOTS = 256                # per-engine ring of RegistrationResults (b2s_scan_result_fetch)
+DUMP_BYTES = 64 << 20             # --dump-outputs writes at most this much
+DUMP_MAP_SAMPLE = 16384           # map points per chain in the dump (fewer when DUMP_BYTES would be exceeded)
 
 
 def env_int(name, default):
@@ -206,6 +212,32 @@ def cpu_baseline_sample(lp, ratio, n_sample):
 # ----------------------------------------------------------------------------------------------------------------------
 # GPU arm
 # ----------------------------------------------------------------------------------------------------------------------
+def dump_last_step(out_dir, maps, last_slot, scans, suffix=""):
+    """Writes what the timed path returned in its last step, as float64 .npy files: every chain's RegistrationResult for each of
+    the step's `scans` scans (shape chains x scans ...), every chain's submap pose and size, and a seeded sample of every chain's
+    map.  The map is sorted before sampling, so the sample does not depend on the order the device stores the points in."""
+    res = [[m.fetchResult((last_slot[c] - scans + 1 + j) % RESULT_SLOTS) for j in range(scans)] for c, m in enumerate(maps)]
+    out = {"transformation": np.array([[r.transformation_ for r in rc] for rc in res]),
+           "fitness": np.array([[r.fitness_ for r in rc] for rc in res]),
+           "inlier_rmse": np.array([[r.inlier_rmse_ for r in rc] for rc in res]),
+           "n_corr": np.array([[r.n_corr for r in rc] for rc in res], dtype=np.float64),
+           "iters": np.array([[r.iters for r in rc] for rc in res], dtype=np.float64),
+           "pose": np.array([m.submap.getPose() for m in maps]),
+           "map_size": np.array([m.submap.size() for m in maps], dtype=np.float64)}
+    clouds = [m.submap.getMapPointCloud() for m in maps]
+    budget = DUMP_BYTES - sum(a.nbytes for a in out.values())
+    n_pick = min([DUMP_MAP_SAMPLE, max(0, budget) // (48 * len(maps))] + [len(x) for x, _ in clouds])
+    xs, ns = [], []
+    for x, n in clouds:
+        order = np.lexsort((n[:, 2], n[:, 1], n[:, 0], x[:, 2], x[:, 1], x[:, 0]))
+        pick = order[np.sort(np.random.default_rng(0).choice(len(x), size=n_pick, replace=False))]
+        xs.append(x[pick]); ns.append(n[pick])
+    out["map_xyz_sample"] = np.array(xs); out["map_normals_sample"] = np.array(ns)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
 def run_b2s_arm(args):
     import torch
     import torch.distributed as dist
@@ -334,6 +366,8 @@ def run_b2s_arm(args):
     barrier()
     clocks = sampler.stop() if rank == 0 else None
     launches = sum(e.launches for e in engs[:chains]) - l0
+    if args.dump_outputs:   # before the sweep and e2e runs below overwrite the result rings
+        dump_last_step(args.dump_outputs, maps[:chains], slot_log, S, f"_rank{rank}" if world > 1 else "")
     ms_total = max_over_ranks(float(np.sum(step_ms)))
     value = world * chains * K * S / (ms_total * 1e-3)
     # the last scan of every chain: iterations, source size, sanity against ground truth
@@ -528,7 +562,13 @@ def main():
     ap.add_argument("--host-threads", type=int, default=0, help="host threads issuing the chains' launches (0 = auto: 1 with graph replay, 8 eager)")
     ap.add_argument("--no-graph", action="store_true", help="launch every kernel eagerly instead of replaying one CUDA graph per scan")
     ap.add_argument("--nn-cell", type=float, default=0.0, help="NN grid cell edge in metres (0 = max_corr_dist / 4)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the last step's registration results, poses and a map sample to DIR/*.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b2s":
+        ap.error("--dump-outputs writes the GPU arm's outputs (--impl b2s)")
+    if args.dump_outputs and args.scans_per_step > RESULT_SLOTS:
+        ap.error(f"--dump-outputs keeps the last {RESULT_SLOTS} results per chain: --scans-per-step must not exceed that")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

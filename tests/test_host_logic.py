@@ -1,4 +1,5 @@
-"""CPU tests of the host-side mirror (parameter mapping, factories, error behaviour) and of bench.py's helpers."""
+"""CPU tests of the host-side mirror (parameter mapping, factories, error behaviour) and of bench.py's helpers; one -m gpu run
+of bench.py's output dump."""
 import os
 import sys
 
@@ -86,6 +87,32 @@ def test_bench_reference_arm_smoke():
     cfg = bench.make_config(ns)
     assert cfg == line["config"] or {k: v for k, v in cfg.items() if k != "chains_per_gpu"} == {k: v for k, v in line["config"].items() if k != "chains_per_gpu"}
     assert set(cfg) == set(line["config"])
+
+
+@pytest.mark.gpu
+def test_bench_dump_outputs(tmp_path):
+    """bench.py --dump-outputs (small run): the last timed step's results of every chain and scan, poses, map sizes and a map
+    sample, float64, within 64 MB, and consistent with what the JSON line reports about the same step."""
+    import json
+    import subprocess
+    chains, steps, spp = 2, 2, 4
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--chains", str(chains), "--steps", str(steps), "--warmup", "3",
+                          "--scans-per-step", str(spp), "--no-extras", "--no-sweep", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=900)
+    assert out.returncode == 0, out.stderr[-2000:]
+    line = json.loads(out.stdout.strip().splitlines()[-1])
+    assert line["steps"] == steps
+    d = {f[:-4]: np.load(tmp_path / f) for f in os.listdir(tmp_path)}
+    assert sum(os.path.getsize(tmp_path / f) for f in os.listdir(tmp_path)) <= 64 << 20
+    assert all(a.dtype == np.float64 for a in d.values())
+    assert d["transformation"].shape == (chains, spp, 4, 4) and d["pose"].shape == (chains, 4, 4)
+    for k in ("fitness", "inlier_rmse", "n_corr", "iters"):
+        assert d[k].shape == (chains, spp)
+    assert d["map_xyz_sample"].shape == d["map_normals_sample"].shape and d["map_xyz_sample"].shape[:2] == (chains, 16384)
+    obs = line["observed"]
+    assert d["fitness"][:, -1].min() == obs["min_fitness_last_scan"] and int(d["map_size"].mean()) == obs["map_points"]
+    acc = d["fitness"][:, -1] >= 0.7                    # fitness gate passed: the chain's pose is that scan's result
+    assert acc.any() and np.array_equal(d["transformation"][acc, -1], d["pose"][acc])
 
 
 def test_reference_side_shim_type_checks():
